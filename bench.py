@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (oracle port), rank 0
+    python bench.py ... --dump-outputs DIR                    # also write the timed path's last-step outputs as .npy
 
 A "step" is one optimizer step of `Solver.fit` on one batch: fused kernel (sample/read points, forward
 jets, residual, MSE, backward) + all-reduce (N>1) + Adam + loss record.  Workload = BASELINE.json
@@ -305,6 +306,18 @@ class Timed:
                 'paths': 'pinn_step_allreduce (NVLink peer memory, in-kernel) vs pinn_step + NCCL all_reduce'}
 
 
+def dump_outputs(t, outdir):
+    """ What the timed path hands its caller after its last step, as DIR/<name>.npy (float32): the updated flat
+    parameters, the gradient that step applied and its loss.  Inputs are seeded, so two builds run with the same
+    arguments can be compared output for output. """
+    eng = t.eng
+    torch.cuda.synchronize()
+    os.makedirs(outdir, exist_ok=True)
+    for name, v in (('params', eng.flat), ('grads', eng.out[:eng.n_params]),
+                    ('loss', eng.out[eng.n_params:eng.n_params + 1])):
+        np.save(os.path.join(outdir, name + '.npy'), v.detach().cpu().numpy().astype(np.float32))
+
+
 def roofline_blocks(t, kern_ms, step_ms, clk, peaks, workload):
     """ roofline of the fused kernel: the binding roof (FP32 FMA for the thread kernel, tensor cores for the tile
     kernel) first, the HBM fraction BASELINE.json asks for beside it. """
@@ -355,6 +368,8 @@ def main():
     ap_.add_argument('--no-e2e', action='store_true')
     ap_.add_argument('--no-extras', action='store_true', help='skip strong_cfg5 / other_configs')
     ap_.add_argument('--reps', type=int, default=10, help='repetitions of the K-step timed region (min/median/max)')
+    ap_.add_argument('--dump-outputs', metavar='DIR', default=None,
+                     help='after the timed steps, write what their last step computed to DIR/<name>.npy')
     args = ap_.parse_args()
     K, W = args.steps, max(args.warmup, 3)
     rank = int(os.environ.get('RANK', '0'))
@@ -403,6 +418,8 @@ def main():
     ms_total = ms_sorted[len(ms_sorted) // 2]                       # median of the repetitions
     value = gbatch * K / (ms_total * 1e-3)
     last_loss = float(eng.out[eng.n_params].item())
+    if args.dump_outputs and rank == 0:                             # before the runs below advance the parameters
+        dump_outputs(t, args.dump_outputs)
 
     # ---------------- in-kernel sampling variant (the default `fit(sampler=None)` mode) ----------------
     sampled_value = None

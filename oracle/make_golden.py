@@ -125,6 +125,29 @@ def main():
         np.savez_compressed(path, **out)
         print('%-12s B=%-4d P=%-6d loss=%.6e  |grad|=%.4e  -> %s' % (
             name, pts.shape[0], params.size, loss, float(np.linalg.norm(grads)), os.path.relpath(path, ROOT)))
+    if not only or 'reshape_and_concat' in only:
+        reshape_and_concat(outdir)
+
+
+def reshape_and_concat(outdir):
+    """ The reference's `Solver.reshape_and_concat` on P.reshape_and_concat_cases(): per case whether it raised,
+    the output shape, and the values (fp64, concatenated). """
+    cases = P.reshape_and_concat_cases()
+    rejected, shapes, values = [], [], []
+    for args in cases:
+        try:
+            want = ref.Solver.reshape_and_concat(list(args))
+        except Exception:                                  # noqa: BLE001  (the reference rejects the mix)
+            rejected.append(True)
+            shapes.append((0, 0))
+            continue
+        rejected.append(False)
+        shapes.append(tuple(want.shape))
+        values.append(want.detach().to(torch.float64).reshape(-1).numpy())
+    path = os.path.join(outdir, 'reshape_and_concat.npz')
+    np.savez_compressed(path, rejected=np.asarray(rejected), shapes=np.asarray(shapes, dtype=np.int64),
+                        values=np.concatenate(values))
+    print('reshape_and_concat: %d cases, %d rejected -> %s' % (len(cases), sum(rejected), os.path.relpath(path, ROOT)))
 
 
 if __name__ == '__main__':

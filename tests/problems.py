@@ -347,3 +347,31 @@ def bind(name, D, V):
     """ Equation callable with the reference signature `equation(u, *xs)`. """
     eq = PROBLEMS[name]['equation']
     return lambda u, *xs: eq(u, *xs, D=D, V=V)
+
+
+def reshape_and_concat_cases(n_cases=200, seed=0):
+    """ Deterministic argument mixes for `Solver.reshape_and_concat` (how `predict` and constraints read numbers /
+    arrays / lists / tensors): a list of argument lists. """
+    rng = np.random.RandomState(seed)
+    cases = []
+    for _ in range(n_cases):
+        n = int(rng.choice([1, 2, 5, 16]))
+        args = []
+        for _ in range(int(rng.randint(1, 5))):
+            kind = int(rng.randint(7))
+            if kind == 0:
+                args.append(float(np.round(rng.uniform(-3, 3), 3)))
+            elif kind == 1:
+                args.append(int(rng.randint(-3, 4)))
+            elif kind == 2:
+                args.append(rng.uniform(-1, 1, size=n).astype(np.float32))
+            elif kind == 3:
+                args.append(rng.uniform(-1, 1, size=(n, 1)))
+            elif kind == 4:
+                args.append(list(np.round(rng.uniform(-1, 1, size=n), 3)))
+            elif kind == 5:
+                args.append(torch.tensor(rng.uniform(-1, 1, size=n), dtype=torch.float32))
+            else:
+                args.append(torch.tensor(rng.uniform(-1, 1, size=(n, 1)), dtype=torch.float32))
+        cases.append(args)
+    return cases

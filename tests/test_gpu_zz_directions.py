@@ -68,9 +68,12 @@ def test_ragged_batches_against_oracle(n):
     prob = oracle_problem('hess3d', torch.float32, g['params'])
     pts = P.make_points('hess3d', n, seed=77)
     loss, grads, residual = solver.loss_and_grads(pts)
-    l, r, gr = prob.loss_and_grads(pts)
+    l, _, gr = prob.loss_and_grads(pts)
     assert abs(loss - l) <= 1e-5 * abs(l)
-    assert rel_l2(residual.cpu().numpy(), r) <= 1e-5
+    # the residual against fp64: the fp32 oracle's nested autograd is itself 3.6e-5 (rel-L2) off fp64 at n=4097,
+    # one point carrying an error of 2.3e-4
+    _, r64, _ = oracle_problem('hess3d', torch.float64, g['params'].astype(np.float64)).loss_and_grads(pts.astype(np.float64))
+    assert rel_l2(residual.cpu().numpy(), r64) <= 1e-5
     assert rel_l2(grads.cpu().numpy(), gr.numpy()) <= 1e-4
 
 
